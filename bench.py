@@ -10,13 +10,15 @@ Workloads (BASELINE.json):
           `run_inference.py configs/inference_training_sample2.pbtxt` on a 250^3 bounding box, i.e.
           Canvas.segment_all with PolicyPeaks seeds and the pbtxt's inference options, ConvStack3DFFNModel depth 12,
           fov 33^3, deltas 8, FIB-25 weights, on the synthetic stand-in for training_sample2 (Voronoi phantom,
-          seed 0; SURVEY.md 8d).  ONE timed pass = the whole canvas (~25.6 k FoV steps, ~585 objects): a flood
-          fill has no meaningful K-step prefix (seed policy, object commits and the last objects are part of
-          the metric), so --steps is IGNORED for sizing (profiler runs cap the seed list with --max-seeds);
-          `steps` in the output line is the number of FoV steps done.
+          seed 0; SURVEY.md 8d).  ONE timed step = the whole canvas (~25.6 k FoV steps, ~585 objects) on a fresh
+          canvas: a flood fill has no meaningful K-FoV-step prefix (seed policy, object commits and the last objects
+          are part of the metric), so --steps K times K such steps (profiler runs cap the seed list with
+          --max-seeds); `steps` in the output line is K, `fov_steps` the FoV steps done in them.
           `value` = FoV steps / wall clock of segment_all (device PolicyPeaks included) with the volume resident
-          in HBM; `e2e` = the same metric through Runner.run (volume file -> pinned H2D -> segment_all -> D2H ->
-          seg-*.npz / .prob written), which is what a user of run_inference.py gets.
+          in HBM, summed over the K steps; `e2e` = the same metric through one Runner.run (volume file -> pinned
+          H2D -> segment_all -> D2H -> seg-*.npz / .prob written), which is what a user of run_inference.py gets.
+          --dump-outputs DIR writes what the last timed step returned (see dump_outputs); the inputs (volume,
+          weights, PolicyPeaks tie-break noise) are seeded, so two builds can be compared output for output.
   N > 1   configs[3] — a 1024^3 volume as 8 slabs of 512^3 (2x2x2), slabs_of_rank(8, rank, N) per GPU, every slab an
           independent canvas (the reference's subvolume semantics, doc/manual.md:107-127), then the merge inside the
           timed region: all_gather of the id counts, id offsets on the device, NCCL gather of the label AND
@@ -354,6 +356,33 @@ def parity_fields(engine, eng, _lib):
   return out
 
 
+DUMP_SAMPLE_VOXELS = 1 << 20
+
+
+def dump_outputs(out_dir, canvas, _lib, seeds, origins, overlaps):
+  """Writes what the last timed segment_all returned to its caller, as float32 / float64 .npy files (~17 MB):
+  the seeds it was given, origins (id, z, y, x, iters) and overlaps (id, other_id, count) sorted by row, and the
+  labels and quantized probabilities at a fixed sample of voxels (RandomState(0), flat C-order indices)."""
+  os.makedirs(out_dir, exist_ok=True)
+  seg = canvas.read(_lib.ARRAY_SEGMENTATION).ravel()
+  qprob = canvas.read(_lib.ARRAY_QPROB).ravel()
+  index = np.sort(np.random.RandomState(0).choice(seg.size, min(DUMP_SAMPLE_VOXELS, seg.size), replace=False))
+
+  def rows(a, width):
+    a = np.asarray(a, dtype=np.float64).reshape(-1, width)
+    return a[np.lexsort(a.T[::-1])]
+  arrays = {
+      'seeds': np.asarray(seeds, dtype=np.float32).reshape(-1, 3),
+      'origins': rows([(o.id, *o.start_zyx, o.iters) for o in origins], 5),
+      'overlaps': rows([(v.id, v.other_id, v.count) for v in overlaps], 3),
+      'sample_index': index.astype(np.float64),
+      'segmentation': seg[index].astype(np.float32),
+      'qprob': qprob[index].astype(np.float32),
+  }
+  for name, a in arrays.items():
+    np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def run_n1(args, rank, local_rank):
   import torch
   from ffn_b200 import _lib
@@ -376,31 +405,43 @@ def run_n1(args, rank, local_rank):
   warm.segment_all(wseeds[:max(8 * max(args.warmup, 3), 24)])
   warm.close()
 
-  # ---- device-resident leg: the volume is in HBM before the timed region starts
-  canvas = eng.DeviceCanvas(engine, pinned.numpy(), opts, 128.0, 33.0, keep_probability_maps=True)
+  # ---- device-resident leg: --steps timed steps, each one whole segment_all on a fresh canvas whose volume is
+  # in HBM before its step starts; the wall clock sums the steps
   sampler = ClockSampler(local_rank)
   sampler.start()
   sampler.wait_ready()
-  torch.cuda.synchronize()
   launches0 = engine.info()['launches']
-  t0 = time.perf_counter()
-  seeds, _ = device_seeds(canvas)
-  t_seed = time.perf_counter() - t0
-  if seed_cap:
-    seeds = seeds[:seed_cap]
-  origins, _, ctr = canvas.segment_all(seeds, overlaps_cap=max(64 * len(seeds), 1 << 16))
-  torch.cuda.synchronize()
-  wall = time.perf_counter() - t0
+  wall = t_seed = dev_seconds = 0.0
+  steps = vox = 0
+  spec = {}
+  canvas = None
+  for _ in range(args.steps):
+    if canvas is not None:
+      canvas.close()
+    canvas = eng.DeviceCanvas(engine, pinned.numpy(), opts, 128.0, 33.0, keep_probability_maps=True)
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    seeds, _ = device_seeds(canvas)
+    t_seed += time.perf_counter() - t0
+    if seed_cap:
+      seeds = seeds[:seed_cap]
+    origins, overlaps, ctr = canvas.segment_all(seeds, overlaps_cap=max(64 * len(seeds), 1 << 16))
+    torch.cuda.synchronize()
+    wall += time.perf_counter() - t0
+    steps += int(ctr.inference_calls)
+    vox += int(ctr.voxels_segmented)
+    dev_seconds += float(ctr.device_seconds)
+    for k, v in canvas.spec_stats().items():
+      spec[k] = v if k == 'chains' else spec.get(k, 0) + v
   clocks = sampler.stop()
-  launches = engine.info()['launches'] - launches0 + 10        # + the ten seed-policy kernels
-  spec = canvas.spec_stats()
-  steps = int(ctr.inference_calls)
-  dev_seconds = float(ctr.device_seconds)
+  launches = engine.info()['launches'] - launches0 + 10 * args.steps        # + the ten seed-policy kernels per step
+  if args.dump_outputs:
+    dump_outputs(args.dump_outputs, canvas, _lib, seeds, origins, overlaps)
   canvas.close()
 
   # ---- end-to-end leg: what run_inference.py does — Runner.start + Runner.run on a volume file
   if args.skip_e2e:
-    e2e_seconds, e2e_steps, e2e_vox = wall, steps, int(ctr.voxels_segmented)
+    e2e_seconds, e2e_steps, e2e_vox = wall, steps, vox
   else:
     from ffn.inference import runner as runner_mod
     tmp = tempfile.mkdtemp(prefix='ffn_bench_')
@@ -427,18 +468,19 @@ def run_n1(args, rank, local_rank):
   executed = spec['steps_executed'] / dev_seconds * flops_per_step() / 1e12
   line = {
       'metric': 'fov_steps_per_sec', 'value': value, 'unit': 'FoV steps/s', 'n_gpus': 1,
-      'steps': steps, 'warmup': max(args.warmup, 3), 'ms_per_step': 1e3 * wall / max(steps, 1),
+      'steps': args.steps, 'warmup': max(args.warmup, 3), 'ms_per_step': 1e3 * wall / args.steps,
+      'fov_steps': steps, 'ms_per_fov_step': 1e3 * wall / max(steps, 1),
       'higher_is_better': True, 'scaling': 'weak', 'vs_baseline': None,
       'dtype': {'fp16': 'f16', 'fp32': 'f32', 'x2': 'f16x2 (hi+lo split, ~f32)'}[args.compute], 'data': 'synthetic',
       'config': {
           'workload': WORKLOAD_N1,
-          'weights': wdesc, 'accumulate': 'f32', 'timed_pass': 'one whole segment_all (device PolicyPeaks + flood fill + commits); '
-          '--steps is ignored (a flood fill has no meaningful K-step prefix)' + (' — capped at %d seeds' % seed_cap if seed_cap else ''),
+          'weights': wdesc, 'accumulate': 'f32', 'timed_pass': 'each step is one whole segment_all (device PolicyPeaks + flood fill + commits) '
+          'on a fresh canvas' + (' — capped at %d seeds' % seed_cap if seed_cap else ''),
           'l2': 'canvas state (image u8 + 4 seed f32 arrays + segmentation i32 + qprob u8 = 330 MB) exceeds L2; '
                 'the ~25 MB activation working set of four chains is L2-resident by design',
           'published_reference_p100': {'fov_steps_per_sec': 65.5, 'voxels_per_sec': 35216},
       },
-      'voxels_per_sec': float(ctr.voxels_segmented) / wall,
+      'voxels_per_sec': vox / wall,
       'segments': int(ctr.segments), 'objects_run': int(ctr.segment_at_calls), 'seeds': int(len(seeds)),
       'seed_policy_seconds': t_seed,
       'device_only': {'value': kernel_rate, 'unit': 'FoV steps/s', 'seconds': dev_seconds,
@@ -635,7 +677,8 @@ def run_multi(args, rank, local_rank, world):
 def main():
   ap = argparse.ArgumentParser()
   ap.add_argument('--gpus', type=int, default=1)
-  ap.add_argument('--steps', type=int, default=0)
+  ap.add_argument('--steps', type=int, default=0,
+                  help='timed steps: N = 1, whole segment_all passes (0 = one); --impl reference, FoV steps (0 = 24)')
   ap.add_argument('--warmup', type=int, default=3)
   ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
   ap.add_argument('--compute', default='fp16', choices=['fp16', 'fp32', 'x2'])
@@ -646,14 +689,20 @@ def main():
   ap.add_argument('--cpu-baseline-steps', type=int, default=24)
   ap.add_argument('--skip-extras', action='store_true', help='no single-seed / predict / cpu_baseline legs (profiler runs)')
   ap.add_argument('--skip-e2e', action='store_true', help='no Runner.run leg (profiler runs; the line then repeats the device-resident value)')
+  ap.add_argument('--dump-outputs', metavar='DIR', help='N = 1: write what the last timed step computed to DIR/<name>.npy')
   args = ap.parse_args()
   rank = int(os.environ.get('RANK', '0'))
   local_rank = int(os.environ.get('LOCAL_RANK', '0'))
   world = int(os.environ.get('WORLD_SIZE', '1'))
+  if args.steps < 0:
+    ap.error('--steps must be >= 0')
+  if args.dump_outputs and (args.impl == 'reference' or world > 1):
+    ap.error('--dump-outputs is only supported by the N = 1 GPU arm')
 
   if args.impl == 'reference':
     reference_arm(args, rank)
     return
+  args.steps = args.steps or 1
 
   import torch
   import torch.distributed as dist

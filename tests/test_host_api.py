@@ -420,21 +420,27 @@ def test_bench_traffic_comes_from_committed_ncu_capture():
   assert 1e4 < t['bytes_per_step'] < 431244 * 2
 
 
-def test_load_segmentation_reads_the_reference_shipped_result(tmp_path):
+def test_load_segmentation_reads_the_reference_shipped_result(tmp_path, golden_dir):
   """results/fib25/sample-training2.npz of the reference checkout: a Python-2 pickle of OriginInfo under the
-  original module path — storage.load_segmentation reads it (latin1 + module mapping).  Skipped where the
-  reference checkout is absent (the GPU box)."""
-  import shutil
-  import pytest
+  original module path — storage.load_segmentation reads it (latin1 + module mapping).  The file is rebuilt from
+  sample_training2_ref.npz (tests/golden/make_golden_reference_files.py): its `origins` member verbatim, and its
+  labels at a seeded sample of voxels and at every origin's start (0 elsewhere)."""
+  import io
+  import zipfile
   from ffn.inference import storage
-  src = '/root/reference/results/fib25/sample-training2.npz'
-  if not os.path.exists(src):
-    pytest.skip('reference checkout not present')
+  r = np.load(os.path.join(golden_dir, 'sample_training2_ref.npz'))
+  labels = np.zeros(tuple(r['shape']), dtype=np.dtype(str(r['dtype'])))
+  labels.ravel()[r['sample_index']] = r['sample_labels']
+  buf = io.BytesIO()
+  np.save(buf, labels)
   d = tmp_path / '0' / '0'
   d.mkdir(parents=True)
-  shutil.copy(src, str(d / 'seg-0_0_0.npz'))
+  with zipfile.ZipFile(str(d / 'seg-0_0_0.npz'), 'w', zipfile.ZIP_DEFLATED) as z:
+    z.writestr('segmentation.npy', buf.getvalue())
+    z.writestr('origins.npy', r['origins_npy'].tobytes())
   seg, origins = storage.load_segmentation(str(tmp_path), (0, 0, 0))
   assert seg.shape == (250, 250, 250) and seg.dtype == np.uint64
+  np.testing.assert_array_equal(seg.ravel()[r['sample_index']], r['sample_labels'])
   assert len(origins) == 254 and origins[1].iters == 1884
   assert all(seg[tuple(int(v) for v in o.start_zyx)] == sid for sid, o in origins.items())   # every origin carries its own id
 

@@ -94,17 +94,41 @@ def test_toy_flood_fill_bit_exact(golden_dir):
   _check_canvas(canvas, g, exact_seed=True)
 
 
+def _rebuild_fib25_checkpoint(golden_dir, out_dir):
+  """The reference's FIB-25 TF checkpoint, byte for byte: its `.index` and non-weight tensor bytes from fib25_ckpt.npz,
+  the seed_update weights from fib25_convstack.npz placed where the index says (make_golden_reference_files.py)."""
+  import hashlib
+  from ffn_b200 import tf_checkpoint
+  c = _load(golden_dir, 'fib25_ckpt.npz')
+  prefix = os.path.join(str(out_dir), 'model.ckpt-27465036')
+  with open(prefix + '.index', 'wb') as f:
+    f.write(c['index'].tobytes())
+  data = bytearray(int(c['data_size']))
+  pos = 0
+  for lo, hi in c['other_offsets']:
+    data[lo:hi] = c['other_bytes'][pos:pos + hi - lo].tobytes()
+    pos += hi - lo
+  w, b = tf_checkpoint.load_convstack_npz(os.path.join(golden_dir, 'fib25_convstack.npz'))
+  names = ['conv%d_%s' % (i, s) for i in range(12) for s in 'ab'] + ['conv_lom']
+  entries = tf_checkpoint.list_variables(prefix)
+  for name, wi, bi in zip(names, w, b):
+    for kind, arr in (('weights', wi), ('biases', bi)):
+      e = entries['seed_update/%s/%s' % (name, kind)]
+      assert tuple(e['shape']) == arr.shape and e['size'] == arr.nbytes, (name, kind)
+      data[e['offset']:e['offset'] + e['size']] = arr.astype('<f4').tobytes()
+  assert hashlib.sha256(data).hexdigest() == str(c['data_sha256'])
+  with open(prefix + '.data-00000-of-00001', 'wb') as f:
+    f.write(data)
+  return prefix
+
+
 @pytest.mark.slow
-def test_real_net_flood_fill(golden_dir):
-  """Same loop with the FIB-25 conv stack (torch CPU).  Exactness is qualified by the decision
-  margin because conv3d rounding may differ between CPUs."""
-  ckpt = os.environ.get('FFN_CKPT', '/root/reference/models/fib25/model.ckpt-27465036')
-  if not os.path.exists(ckpt + '.index'):
-    ckpt = os.path.join(golden_dir, 'fib25', 'model.ckpt-27465036')
-  if not os.path.exists(ckpt + '.index'):
-    pytest.skip('FIB-25 checkpoint not available')
+def test_real_net_flood_fill(golden_dir, tmp_path):
+  """Same loop with the FIB-25 conv stack (torch CPU), weights read from the TF checkpoint.  Exactness is
+  qualified by the decision margin because conv3d rounding may differ between CPUs."""
   from ffn_b200 import tf_checkpoint
   from oracle.network import ConvStackOracle
+  ckpt = _rebuild_fib25_checkpoint(golden_dir, tmp_path)
   g = _load(golden_dir, 'flood_fill_64.npz')
   w, b = tf_checkpoint.load_convstack_weights(ckpt, 12)
   image = (g['volume'].astype(np.float32) - 128.0) / 33.0
