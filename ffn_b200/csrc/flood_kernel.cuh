@@ -410,13 +410,15 @@ __device__ __forceinline__ void quad_sync(int quad) {   // the four epilogue war
 //   EPI_B_FIRST  conv0_b             : net = v + b            ; out = relu(net)   (:39) starts the residual stream
 //   EPI_B        conv{i}_b, i >= 1   : net = v + b + residual ; out = relu(net)   (:46-49)
 //   EPI_LAST     the final "_b"      : as EPI_B, then logits = seed + b_lom + <relu(net), w_lom> (:51-54, model.py:176-177)
+//   EPI_LAST0    conv0_b at depth 1  : net = v + b, then the logits of EPI_LAST (no residual module: there is no
+//                                      residual stream to read)
 // The fp32 residual stream lives in this thread's TMEM lane, columns behind the accumulator ring
 // (32 columns per tile and chain).
 // Accumulator row m of a tile holds, for the FoV row u = tile_row0 - 1 + m,
 //   D[u][dx*32 + co] = sum_{dz,dy,ci} act[u + dz*pp + dy*xp][ci] * W[dz,dy,dx][ci][co]
 // and the convolution output is out[v] = D[v-1][dx=-1] + D[v][dx=0] + D[v+1][dx=+1]: one lane up /
 // down, done with warp shuffles (+ a 2 KB shared-memory exchange at the three warp boundaries).
-enum EpiKind : int { EPI_A = 0, EPI_B_FIRST = 1, EPI_B = 2, EPI_LAST = 3 };
+enum EpiKind : int { EPI_A = 0, EPI_B_FIRST = 1, EPI_B = 2, EPI_LAST = 3, EPI_LAST0 = 4 };
 
 template <int KIND, bool X2 = false>
 __device__ __forceinline__ int tc_epilogue(Ctx& c, int k, int layer, int ntiles) {
@@ -426,6 +428,7 @@ __device__ __forceinline__ int tc_epilogue(Ctx& c, int k, int layer, int ntiles)
   constexpr float kUnscale = 1.0f / (float)(1 << kSplitShift);   // X2: accumulators carry w * 2^kSplitShift
   constexpr bool kReadRes = KIND == EPI_B || KIND == EPI_LAST;
   constexpr bool kWriteRes = KIND == EPI_B_FIRST || KIND == EPI_B;
+  constexpr bool kLast = KIND == EPI_LAST || KIND == EPI_LAST0;
   const int half = c.warp >> 2, wq = c.warp & 3;
   const float4* bias4 = reinterpret_cast<const float4*>(c.s_bias + layer * 32 + half * 16);   // re-read per tile: 16 registers less
   const size_t chunk_stride = (size_t)g.rows_alloc * 8;
@@ -519,7 +522,7 @@ __device__ __forceinline__ int tc_epilogue(Ctx& c, int k, int layer, int ntiles)
       for (int q = 0; q < 16; ++q) rr[q] = __float_as_uint(v[q]);
       sm100::tmem_st16(tres, rr);
     }
-    if (KIND != EPI_LAST) {
+    if (!kLast) {
       if (valid) {
         // out = relu(.) as fp16: the ReLU rides on the conversion (cvt.rn.relu.f16x2.f32)
         __half* dst = out_base + (size_t)r * 8;   // [k-chunk][row][8 halfs]; this half owns chunks 2*half, 2*half+1
@@ -728,7 +731,7 @@ __device__ __forceinline__ void layers_pipelined(Ctx& c, unsigned mask) {
       for (int k = 0; k < kMaxChains; ++k) {
         if (!((mask >> k) & 1u)) continue;
         if (last) {
-          const int hit = tc_epilogue<EPI_LAST>(c, k, layer, ntiles);
+          const int hit = layer == 1 ? tc_epilogue<EPI_LAST0>(c, k, layer, ntiles) : tc_epilogue<EPI_LAST>(c, k, layer, ntiles);
           publish_counts(c, k, hit);          // the round ends with a grid barrier: no chain arrival needed
         } else {
           if (!(layer & 1)) {
@@ -846,7 +849,7 @@ __device__ __forceinline__ void tc_layer_x2(Ctx& c, int layer) {
     }
   } else if (c.warp < 8) {
     if (last) {
-      hit = tc_epilogue<EPI_LAST, true>(c, 0, layer, ntiles);
+      hit = layer == 1 ? tc_epilogue<EPI_LAST0, true>(c, 0, layer, ntiles) : tc_epilogue<EPI_LAST, true>(c, 0, layer, ntiles);
     } else if (!(layer & 1)) {
       tc_epilogue<EPI_A, true>(c, 0, layer, ntiles);
     } else if (layer == 1) {

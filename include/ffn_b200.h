@@ -114,7 +114,12 @@ const char* ffn_last_error(void);
 /* ---- engine: owns device context, packed weights, workspace ------------------------------
  * Replaces Runner._init_tf_model + Saver.restore (ffn/inference/runner.py:98-163).
  * weights_dhwio[i]: float32 [3,3,3,Cin,32] in TF DHWIO order for i < 2*depth (Cin = 2 for i == 0),
- * weights_dhwio[2*depth]: conv_lom [1,1,1,32,1]; biases[i]: [32] (conv_lom: [1]). */
+ * weights_dhwio[2*depth]: conv_lom [1,1,1,32,1]; biases[i]: [32] (conv_lom: [1]).
+ * Geometry limits (an error, not a crash, when exceeded): every FoV size odd and >= 3; x extent <= 33 (the
+ * operand staging of one tile must fit the 227 KB of shared memory: x = 35 needs 233 072 B); depth 1..16;
+ * deltas in [0, fov // 2]; at most 10 tiles of 126 FoV rows per CTA (the fp32 residual stream of every tile lives
+ * in TMEM), i.e. ceil(tiles / SMs) <= 10 — (65,65,33) has 1124 tiles and needs at least 113 SMs.  The more tiles
+ * a CTA owns, the fewer chains fit (ffn_engine_set_chains): 10 / tiles-per-CTA, at most 4. */
 int ffn_engine_create(int device, const FfnModelDesc* model, const float* const* weights_dhwio,
                       const float* const* biases, int compute_mode, FfnEngine** out);
 /* Canvases created from the engine may outlive this call: the engine is then released by the last
